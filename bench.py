@@ -10,6 +10,8 @@ CP+head gradient per step).  Prints ONE JSON line (rank 0).  --config selects th
 (vitl16_r32 / vith14_r32 / vitb16_eval); --global-batch G fixes the GLOBAL batch instead (strong scaling, configs[2]).
 The CPU arm (--impl reference, and cpu_baseline in the default line) is BASELINE configs[0] exactly as BASELINE.md
 section 5 specifies it: ViT-B/16 rank 8 fp32 batch 32, 1 warm-up + best of 3, oracle port, all host threads.
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy; model and batches are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -148,6 +150,35 @@ def apply_weight_dropout(vit, mode):
     wdrop.set_weight_dropout(vit, mode)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(loss, opt):
+    """What a fine-tune step leaves its caller, copied to the host: the loss it returns and every trainable tensor (CP
+    factors and head) after its AdamW update.  Gradients are left out: AdamW's first updates move each element by about
+    lr * sign(g), so elements whose gradient is rounding noise (fp32 atomics) go either way.  Two runs of the default
+    configuration with --steps 20 --warmup 5 on one B200 (1,000 W limit) differed in the last gradient by up to 3e-1
+    relative, in the parameters by at most 1.3e-2 relative and in the loss by 8e-3."""
+    flat = opt.flat.flat.detach().cpu().numpy()
+    out = {"loss": loss.detach().float().cpu().numpy().reshape(1)}
+    for n, p in opt.flat.named:
+        a, b = opt.flat.slices[n]
+        out["param." + n] = flat[a:b].reshape(p.shape)
+    return out
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: one float32 / float64 DIR/<name>.npy per array."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes of outputs exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def _install_init_module():
     """Random-init weights of the architecture + non-default CP factors (the reference's default init makes every
     delta exactly zero, cara.py:128,132; SURVEY D.3 recipe keeps the adapter numerically alive)."""
@@ -244,6 +275,8 @@ def run_cuda(args):
     launches = K.launch_count - launches0
     clocks = sampler.stop() if rank == 0 else None
     loss_value = float(loss)
+    # taken now: the roofline and end-to-end passes below keep training the same model
+    outputs = step_outputs(loss, opt) if args.dump_outputs and rank == 0 else None
 
     # ------------------------------------------------------------ roofline of the dominant kernel: the same step run
     # eagerly with CUDA events around every fused-projection launch (events inside a replayed graph cannot be timed)
@@ -344,6 +377,8 @@ def run_cuda(args):
         if world == 1 and not args.no_cpu_baseline:
             out["cpu_baseline"] = cpu_reference(args, steps=3, warmup=1)
         print(json.dumps(out), flush=True)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         if hasattr(step, "release"):
             step.release()                       # captured collectives must be gone before the communicator is
@@ -392,6 +427,8 @@ def run_eval(args, cfg, vit, dev, world, rank):
     barrier()
     ms = e0.elapsed_time(e1)
     launches = K.launch_count - launches0
+    # the predicted classes of the last timed batch (float64 holds every class index exactly)
+    outputs = {"pred": pred.double().cpu().numpy()} if args.dump_outputs and rank == 0 else None
     stage = [torch.empty_like(dev_x[0]) for _ in range(2)]
     pred_host = torch.zeros(B, dtype=torch.int64).pin_memory()
     copy_stream = torch.cuda.Stream(device=dev)
@@ -439,6 +476,8 @@ def run_eval(args, cfg, vit, dev, world, rank):
                         "traffic": None, "peak_source": peak_src}}
     if rank == 0:
         print(json.dumps(out), flush=True)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
 
@@ -522,7 +561,11 @@ def main():
     ap.add_argument("--global-batch", type=int, default=0,
                     help="strong scaling: fix the GLOBAL batch (BASELINE configs[2]: 2048) and split it over the GPUs")
     ap.add_argument("--no-graph", action="store_true", help="enqueue every step eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl != "reference":
         args.warmup = 3
     if args.impl == "reference":
