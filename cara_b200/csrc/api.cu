@@ -132,8 +132,8 @@ int cara_attn_bwd(const void* qkv, const void* o, const void* o_lo, const float*
   cara::AttnArgs a{static_cast<const bf16*>(qkv), static_cast<bf16*>(const_cast<void*>(o)),
                    static_cast<bf16*>(const_cast<void*>(o_lo)), const_cast<float*>(lse),
                    static_cast<const bf16*>(d_o), static_cast<bf16*>(dqkv), delta_ws, B, N, H, D, scale};
-  if (o == nullptr && (D != 64 || N > 256 || delta_ws == nullptr))
-    return fail(-50, "cara_attn_bwd: a precomputed delta (o == NULL) needs D = 64, N <= 256");
+  if (o == nullptr && (D != 64 || delta_ws == nullptr))
+    return fail(-50, "cara_attn_bwd: a precomputed delta (o == NULL) needs D = 64 and delta_ws");
   CARA_RET(cara::attn_bwd_launch(a, CARA_STREAM(stream)), "cara_attn_bwd");
 }
 int cara_gelu_f32(const float* dy, const float* x, float* out, long n, void* stream) {

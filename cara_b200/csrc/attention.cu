@@ -453,8 +453,8 @@ int bwd_t(const AttnArgs& a, cudaStream_t st) {
 
 }  // namespace
 
-// CARA_ATTN_TC (default 3): bit 0 = tcgen05 forward, bit 1 = tcgen05 backward (D = 64, N <= 256); other shapes and
-// cleared bits run the mma.sync kernels above.
+// CARA_ATTN_TC (default 3): bit 0 = tcgen05 forward, bit 1 = tcgen05 backward (D = 64: attention_tc.cu for N <= 256,
+// the key-tiled kernels of attention_long.cu above); D = 80 and cleared bits run the mma.sync kernels above.
 static int attn_tc_mask() {
   static int v = -1;
   if (v < 0) {
@@ -467,7 +467,8 @@ static int attn_tc_mask() {
 int attn_fwd_launch(const AttnArgs& a, cudaStream_t st) {
   if (a.B <= 0 || a.N <= 0 || a.H <= 0) return -50;
   if (attn_tc_mask() & 1) {
-    const int rc = attn_fwd_tc_launch(a, st);
+    int rc = attn_fwd_tc_launch(a, st);
+    if (rc == 1) rc = attn_fwd_long_launch(a, st);
     if (rc <= 0) return rc;
   }
   if (a.D == 64) return fwd_t<64>(a, st);
@@ -477,12 +478,14 @@ int attn_fwd_launch(const AttnArgs& a, cudaStream_t st) {
 int attn_bwd_launch(const AttnArgs& a, cudaStream_t st) {
   if (a.B <= 0 || a.N <= 0 || a.H <= 0) return -50;
   if (a.o == nullptr) {                                         // delta already in a.delta (EPI_DELTA of the proj dX GEMM)
-    const int rc = (attn_tc_mask() & 2) ? attn_bwd_tc_launch(a, st) : 1;
+    int rc = (attn_tc_mask() & 2) ? attn_bwd_tc_launch(a, st) : 1;
+    if (rc == 1 && (attn_tc_mask() & 2)) rc = attn_bwd_long_launch(a, st);
     return rc == 1 ? -50 : rc;
   }
   if (a.o_lo == nullptr) return -50;
   if (attn_tc_mask() & 2) {
-    const int rc = attn_bwd_tc_launch(a, st);
+    int rc = attn_bwd_tc_launch(a, st);
+    if (rc == 1) rc = attn_bwd_long_launch(a, st);
     if (rc <= 0) return rc;
   }
   if (a.D == 64) return bwd_t<64>(a, st);

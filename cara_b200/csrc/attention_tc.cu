@@ -921,6 +921,12 @@ int attn_bwd_tc_launch(const AttnArgs& a, cudaStream_t st) {
   return launch_pdl_f<2>(attn_bwd_tc_kernel, dim3(grid), dim3(TCB_THREADS), smem, st, map_qkv, map_do, a, npad, qk_pairs) ==
                  cudaSuccess ? 0 : -53;
 }
+// rowsum(dO (.) (O + O_lo)) into a.delta: the pre-pass of the long-sequence backward (attention_long.cu)
+int attn_delta_launch(const AttnArgs& a, cudaStream_t st) {
+  const long rows = static_cast<long>(a.B) * a.N;
+  return launch_pdl_f<2>(attn_delta_kernel, dim3(static_cast<int>((rows + 7) / 8)), dim3(256), 0, st, a.d_o, a.o, a.o_lo,
+                         a.delta, static_cast<int>(rows), a.N, a.H) == cudaSuccess ? 0 : -53;
+}
 int attn_debug_read(long long* out, int n) {
   if (n > 64) n = 64;
   if (n <= 0 || cudaMemcpyFromSymbol(out, g_attn_dbg, sizeof(long long) * n) != cudaSuccess) return 0;

@@ -310,8 +310,8 @@ def attn_fwd(qkv, B, N, H, D, scale, train=True):
 
 def attn_delta_fusable(N, D):
     """Shapes whose softmax-backward row term the output projection's dX GEMM can emit (EPI_DELTA): the tcgen05
-    attention path, head dim = one 64-column epilogue step."""
-    return delta_in_gemm and D == 64 and N <= 256 and (int(os.environ.get("CARA_ATTN_TC", "3")) & 2) != 0
+    attention path (any N), head dim = one 64-column epilogue step."""
+    return delta_in_gemm and D == 64 and (int(os.environ.get("CARA_ATTN_TC", "3")) & 2) != 0
 
 
 def attn_bwd(qkv, o, o_lo, lse, d_o, B, N, H, D, scale, delta=None):

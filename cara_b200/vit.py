@@ -360,6 +360,9 @@ _GEOMETRY = {
     "vit_large_patch16_224_in21k": dict(patch_size=16, embed_dim=1024, depth=24, num_heads=16, num_classes=21843),
     "vit_large_patch16_224": dict(patch_size=16, embed_dim=1024, depth=24, num_heads=16, num_classes=1000),
     "vit_huge_patch14_224_in21k": dict(patch_size=14, embed_dim=1280, depth=32, num_heads=16, num_classes=21843),
+    # fine-tuned at 384 px (577 tokens): attention runs on the key-tiled kernels of csrc/attention_long.cu
+    "vit_base_patch16_384": dict(img_size=384, patch_size=16, embed_dim=768, depth=12, num_heads=12, num_classes=1000),
+    "vit_large_patch16_384": dict(img_size=384, patch_size=16, embed_dim=1024, depth=24, num_heads=16, num_classes=1000),
 }
 
 

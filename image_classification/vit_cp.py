@@ -10,7 +10,8 @@ cosine schedule stepped with the epoch index (vit_cp.py:55-56,187), test every 1
 checkpoint (vit_cp.py:57-68).  Additive flags: ``--epochs``, ``--batch-size``, ``--synthetic`` (VTAB-shaped
 random data when ./data/vtab-1k is absent), ``--no-merge`` (evaluate through the adapter kernels instead of
 folding the CP delta into the frozen weights first), ``--weight-dropout exact|skip`` (default exact = the
-reference's train-mode dropout on the materialised delta), ``--retrain-mode``, ``--allow-random-init``.  Multi-GPU: launch with torchrun; the batch is sharded
+reference's train-mode dropout on the materialised delta), ``--retrain-mode``, ``--allow-random-init``, ``--img-size``
+(fine-tune at another resolution, e.g. 384: the position embedding is resampled and the data resized to match).  Multi-GPU: launch with torchrun; the batch is sharded
 over the ranks and only the flat CP+head gradient (<= 1.1 MB) is all-reduced.
 """
 import os
@@ -27,18 +28,18 @@ from vtab_config import config  # noqa: E402
 
 from cara_b200 import train as T  # noqa: E402
 from cara_b200.merge import merge_cara  # noqa: E402
-from cara_b200.vit import create_model  # noqa: E402
+from cara_b200.vit import _GEOMETRY, create_model  # noqa: E402
 from cara_b200.wdrop import set_weight_dropout  # noqa: E402
 from src.cara.cara import cara  # noqa: E402
 
 
 @th.no_grad()
-def test(model, dl):
+def test(model, dl, img_size=224):
     """Top-1 accuracy (reference vit_cp.py:73-82; avalanche's Accuracy replaced by a running mean)."""
     model.eval()
     correct = total = 0
     for x, y in dl:
-        x, y = to_device(x, y)
+        x, y = to_device(x, y, size=img_size)
         correct += int((model(x).argmax(dim=1).view(-1) == y).sum())
         total += int(y.numel())
     return correct / max(total, 1)
@@ -60,7 +61,7 @@ def train(args, model, dl, tdl, opt, epochs, world_size=1, rank=0):
     step = None
     for epoch in range(epochs):
         for x, y in dl:
-            x, y = to_device(x, y)
+            x, y = to_device(x, y, size=args.img_size)
             if world_size > 1:
                 lo, hi = T.shard_batch(x.shape[0], rank, world_size)
                 x, y = x[lo:hi], y[lo:hi]
@@ -72,7 +73,7 @@ def train(args, model, dl, tdl, opt, epochs, world_size=1, rank=0):
             print(f"e: {epoch}, l: {round(float(loss), 7)}, a:{acc}", flush=True)
         if epoch % 10 == 0 and epoch != 0:
             sched.after_test(epoch)
-            acc = test(model, tdl)
+            acc = test(model, tdl, args.img_size)
             if args.retrain_mode:
                 model.train()
             step = None                       # the mode (dropout / DropPath kernels) is baked into the captured graph
@@ -87,7 +88,7 @@ def train(args, model, dl, tdl, opt, epochs, world_size=1, rank=0):
 
 def build_model(args, data_config, num_classes):
     """vit_cp.py:155-166 of the reference: backbone (+ ./ViT-B_16.npz), cara(), fresh classifier, on the GPU."""
-    vit = create_model(args.model, checkpoint_path="./ViT-B_16.npz", drop_path_rate=0.1,
+    vit = create_model(args.model, checkpoint_path="./ViT-B_16.npz", drop_path_rate=0.1, img_size=args.img_size,
                        allow_missing_checkpoint=args.synthetic or args.allow_random_init)
     vit = cara({"model": vit, "rank": args.dim, "scale": data_config["scale"], "l_mu": data_config["init_mean"],
                 "l_std": data_config["init_std"]})
@@ -128,7 +129,17 @@ def _parse_args(argv=None):
                    help="keep the random initialisation when ./ViT-B_16.npz is missing (implied by --synthetic)")
     p.add_argument("--gpu-preprocess", action="store_true",
                    help="decode on the CPU, resize + normalise on the GPU (bit-identical to the reference's transforms)")
-    return p.parse_args(argv)
+    p.add_argument("--img-size", default=None, type=int,
+                   help="input resolution (default: the model's own, 224 for the *_224 models); a positive multiple "
+                        "of the patch size, e.g. 384 for ViT-B/16 (577 tokens)")
+    args = p.parse_args(argv)
+    geom = _GEOMETRY.get(args.model, {})                  # (an unknown name is reported by create_model)
+    patch = geom.get("patch_size", 16)
+    if args.img_size is None:
+        args.img_size = geom.get("img_size", 224)
+    elif args.img_size <= 0 or args.img_size % patch != 0:
+        p.error("--img-size %d is not a positive multiple of the patch size %d of %s" % (args.img_size, patch, args.model))
+    return args
 
 
 def main(sd=None):
@@ -152,13 +163,14 @@ def main(sd=None):
     th.cuda.manual_seed_all(seed)
 
     train_dl, test_dl = get_data(name, evaluate=True, batch_size=args.batch_size,
-                                 synthetic=True if args.synthetic else None, gpu_preprocess=args.gpu_preprocess)
+                                 synthetic=True if args.synthetic else None, gpu_preprocess=args.gpu_preprocess,
+                                 img_size=args.img_size)
     vit = build_model(args, data_config, get_classes_num(name))
 
     if args.evaluate is not None:
         print("Only evaluation")
         load_for_evaluate(vit, args.evaluate, merge=not args.no_merge)
-        acc = test(vit, test_dl)
+        acc = test(vit, test_dl, args.img_size)
         print(f"Accuracy: {acc}")
         sys.exit(0)
 
@@ -168,7 +180,7 @@ def main(sd=None):
     opt = T.FusedAdamW(T.FlatTrainable(trainable), lr=args.lr, weight_decay=1e-4)
     vit, old_name = train(args, vit, train_dl, test_dl, opt, args.epochs, world, rank)
     print("\n\n Evaluating....")
-    acc = test(vit, test_dl)
+    acc = test(vit, test_dl, args.img_size)
     print(acc)
     if acc > args.best_acc and rank == 0:
         args.best_acc = acc

@@ -40,14 +40,14 @@ class SyntheticImages(torch.utils.data.Dataset):
 
 
 class _FileList(torch.utils.data.Dataset):
-    def __init__(self, root, flist, decode_only=False):
+    def __init__(self, root, flist, decode_only=False, img_size=224):
         from torchvision import transforms
         self.root = root
         self.decode_only = decode_only
         with open(flist) as f:
             self.items = [(p, int(lab)) for p, lab in (ln.split() for ln in f if ln.strip())]
         self.tf = transforms.Compose([
-            transforms.Resize((224, 224), interpolation=transforms.InterpolationMode.BICUBIC),
+            transforms.Resize((img_size, img_size), interpolation=transforms.InterpolationMode.BICUBIC),
             transforms.ToTensor(),
             transforms.Normalize(mean=[0.485, 0.456, 0.406], std=[0.229, 0.224, 0.225])])
 
@@ -72,34 +72,36 @@ def _collate_decoded(batch):
 _PRE = {}
 
 
-def to_device(x, y, device="cuda"):
-    """A loader batch -> (fp32 [B,3,224,224], labels) on the device; decoded uint8 batches go through the GPU
+def to_device(x, y, device="cuda", size=224):
+    """A loader batch -> (fp32 [B,3,size,size], labels) on the device; decoded uint8 batches go through the GPU
     resize / normalise kernels."""
     if isinstance(x, (list, tuple)):
         from cara_b200.preprocess import GpuPreprocessor
         dev = torch.device(device)
         if dev.index is None and dev.type == "cuda":
             dev = torch.device("cuda", torch.cuda.current_device())
-        pre = _PRE.get(dev)
+        pre = _PRE.get((dev, size))
         if pre is None:
-            pre = _PRE[dev] = GpuPreprocessor(dev)
+            pre = _PRE[(dev, size)] = GpuPreprocessor(dev, size=size)
         return pre(x), y.to(dev, non_blocking=True)
     return x.to(device, non_blocking=True), y.to(device, non_blocking=True)
 
 
-def get_data(name, evaluate=True, batch_size=64, synthetic=None, train_len=1000, val_len=512, gpu_preprocess=False):
+def get_data(name, evaluate=True, batch_size=64, synthetic=None, train_len=1000, val_len=512, gpu_preprocess=False,
+             img_size=224):
     root = "./data/vtab-1k/" + name
     if synthetic is None:
         synthetic = not os.path.isdir(root)
     if synthetic:
         print(f"Synthetic VTAB-1k-shaped data for {name} ({root} not used)")
         k = get_classes_num(name)
-        train, val = SyntheticImages(train_len, k, 1), SyntheticImages(val_len, k, 2)
+        train, val = SyntheticImages(train_len, k, 1, img=img_size), SyntheticImages(val_len, k, 2, img=img_size)
         workers = 0
     else:
         print(f"Getting data from root: {root}")
         tr, va = ("/train800val200.txt", "/test.txt") if evaluate else ("/train800.txt", "/val200.txt")
-        train, val = _FileList(root, root + tr, gpu_preprocess), _FileList(root, root + va, gpu_preprocess)
+        train = _FileList(root, root + tr, gpu_preprocess, img_size)
+        val = _FileList(root, root + va, gpu_preprocess, img_size)
         workers = 4
     collate = _collate_decoded if (gpu_preprocess and not synthetic) else None
     train_loader = torch.utils.data.DataLoader(train, batch_size=batch_size, shuffle=True, drop_last=True,
