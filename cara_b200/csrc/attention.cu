@@ -322,12 +322,16 @@ attn_bwd_kernel(const AttnArgs a) {
   const float* lse = a.lse + (static_cast<long>(b) * a.H + h) * N;
   for (int row = tid; row < nstat; row += BWD_THREADS) {
     s_lse[row] = row < N ? lse[row] : 1e30f;
-    s_delta[row] = 0.f;
+    if (row >= N) s_delta[row] = 0.f;
   }
-  __syncthreads();
   {
-    // all threads, 16-byte coalesced loads, two items in flight per thread: the global-latency part of the CTA
-    constexpr int CH = D / 8;
+    // One group of G lanes per row: lane c of the group loads 16-byte chunk c of the row, and the group sums the
+    // chunks with shuffles in a fixed order, so dqkv is bit-identical from run to run (shared-memory atomics from
+    // several warps into one row -- a D = 80 row spans two warps -- add in whatever order the warps arrive).
+    // U rows in flight per group, 32 per pass of the CTA: this loop is the global-latency part of the CTA.
+    constexpr int CH = D / 8, G = CH <= 8 ? 8 : 16, U = G / 4, NG = BWD_THREADS / G;
+    static_assert(CH <= 16, "one row per group of at most 16 lanes");
+    const int c = lane % G, grp = tid / G;
     auto dot8 = [](const uint4& x, const uint4& y, const uint4& z) {
       const uint32_t xw[4] = {x.x, x.y, x.z, x.w}, yw[4] = {y.x, y.y, y.z, y.w}, zw[4] = {z.x, z.y, z.z, z.w};
       float acc = 0.f;
@@ -340,18 +344,26 @@ attn_bwd_kernel(const AttnArgs a) {
       }
       return acc;
     };
-    const int items = N * CH;
-    for (int i0 = tid; i0 < items; i0 += 2 * BWD_THREADS) {
-      const int i1 = i0 + BWD_THREADS;
-      const bool has1 = i1 < items;
-      const int r0 = i0 / CH, c0 = i0 % CH, r1 = has1 ? i1 / CH : r0, c1 = has1 ? i1 % CH : c0;
-      const long o0 = static_cast<long>(r0) * C + c0 * 8, o1 = static_cast<long>(r1) * C + c1 * 8;
-      const uint4 x0 = *reinterpret_cast<const uint4*>(dob + o0), y0 = *reinterpret_cast<const uint4*>(ob + o0),
-                  z0 = *reinterpret_cast<const uint4*>(olb + o0);
-      const uint4 x1 = *reinterpret_cast<const uint4*>(dob + o1), y1 = *reinterpret_cast<const uint4*>(ob + o1),
-                  z1 = *reinterpret_cast<const uint4*>(olb + o1);
-      atomicAdd(&s_delta[r0], dot8(x0, y0, z0));
-      if (has1) atomicAdd(&s_delta[r1], dot8(x1, y1, z1));
+    for (int r0 = 0; r0 < N; r0 += U * NG) {                   // warp-uniform trip count: every lane shuffles
+      uint4 x[U] = {}, y[U] = {}, z[U] = {};
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int r = r0 + u * NG + grp;
+        if (c < CH && r < N) {
+          const long off = static_cast<long>(r) * C + c * 8;
+          x[u] = *reinterpret_cast<const uint4*>(dob + off);
+          y[u] = *reinterpret_cast<const uint4*>(ob + off);
+          z[u] = *reinterpret_cast<const uint4*>(olb + off);
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        float v = dot8(x[u], y[u], z[u]);                         // 0 for idle lanes and rows >= N
+#pragma unroll
+        for (int s = G / 2; s > 0; s >>= 1) v += __shfl_xor_sync(0xffffffffu, v, s);
+        const int r = r0 + u * NG + grp;
+        if (c == 0 && r < N) s_delta[r] = v;
+      }
     }
   }
   cp_async_commit_wait_all();

@@ -145,14 +145,14 @@ CARA_API int cara_adapter_cols(const void* X, long ldx, int M, int Kc, const voi
  * For training also pass lse [B,H,N] fp32 (base-2 log-sum-exp of the scaled scores) and o_lo [B,N,H,D] bf16
  * (the rounding residual of o: o_fp32 = o + o_lo), both consumed by cara_attn_bwd; NULL for inference.
  * D in {64,80}.  D = 64 runs on tcgen05 at every N (N <= 256: one head per CTA pass; N > 256: 128-key tiles);
- * D = 80 runs on mma.sync with the whole head in shared memory (N up to about 600). */
+ * D = 80 runs on mma.sync with the whole head in shared memory: N <= 432, larger N returns an error. */
 CARA_API int cara_attn_fwd(const void* qkv, void* o, void* o_lo, float* lse, int B, int N, int H, int D,
                            float scale, void* stream);
 /* delta_ws: caller-provided fp32 workspace [B,H,N] (rowsum(dO (.) O), written by a streaming pre-pass).
  * o == NULL (D = 64 only, any N): delta_ws already holds it -- written by the output projection's dX GEMM
  * (cara_gemm_cp, epi = CARA_EPI_DELTA) -- and the pre-pass is skipped.
- * D = 64 runs on tcgen05 at every N, without atomics (dqkv is bit-identical from run to run); D = 80 runs on mma.sync
- * with the whole head in shared memory (N up to about 450). */
+ * D = 64 runs on tcgen05 at every N; D = 80 runs on mma.sync with the whole head in shared memory: N <= 320, larger N
+ * returns an error.  Neither uses atomics: dqkv is bit-identical from run to run. */
 CARA_API int cara_attn_bwd(const void* qkv, const void* o, const void* o_lo, const float* lse, const void* d_o,
                            void* dqkv, float* delta_ws, int B, int N, int H, int D, float scale, void* stream);
 /* Profiling aid: copies up to n device-side cycle stamps recorded by the attention kernels (debug builds of the

@@ -9,6 +9,7 @@ import pytest
 import torch
 
 from oracle import cara_oracle as O
+from tests._attn_ref import check
 
 pytestmark = pytest.mark.gpu
 
@@ -20,64 +21,6 @@ D = 64
 def K():
     from cara_b200 import kernels
     return kernels
-
-
-def ref_attention(qkv, d_o, scale):
-    """fp64 forward and backward of softmax(q k^T scale) v, qkv [B,N,3,H,D], d_o [B*N, H*D] ->
-    (o [B,N,H,D], lse [B,H,N] base 2, dqkv [B,N,3,H,D]), one sample at a time."""
-    B, N, _, H, _ = qkv.shape
-    o, lse, dqkv = [], [], []
-    for b in range(B):
-        q, k, v = [t.double() for t in qkv[b].permute(1, 2, 0, 3)]               # [H,N,D]
-        s = (q @ k.transpose(-1, -2)) * scale
-        ls = torch.logsumexp(s, -1)
-        p = torch.exp(s - ls[..., None])
-        ob = p @ v
-        o.append(ob.transpose(0, 1))
-        lse.append(ls / math.log(2.0))
-        if d_o is not None:
-            do = d_o.view(B, N, H, D)[b].double().transpose(0, 1)                   # [H,N,D]
-            dp = do @ v.transpose(-1, -2)
-            ds = p * (dp - (do * ob).sum(-1, keepdim=True))
-            dqkv.append(torch.stack([(ds @ k) * scale, (ds.transpose(-1, -2) @ q) * scale, p.transpose(-1, -2) @ do],
-                                    0).permute(2, 0, 1, 3))
-    return torch.stack(o), torch.stack(lse), (torch.stack(dqkv) if dqkv else None)
-
-
-def worst_head(a, b, head_dim):
-    """max over (sample, head) of the relative L2 error; ``head_dim`` is the index of the head axis of [B, N, (3,) H, D]
-    tensors, or None for lse [B, H, N]."""
-    a, b = a.double(), b.double()
-    if head_dim is None:
-        num = (a - b).norm(dim=-1)
-        den = b.norm(dim=-1)
-    else:
-        a, b = a.movedim(head_dim, 1), b.movedim(head_dim, 1)               # [B, H, N, D]
-        num = (a - b).flatten(2).norm(dim=-1)
-        den = b.flatten(2).norm(dim=-1)
-    return float((num / den.clamp_min(1e-30)).max())
-
-
-def check(K, qkv, B, N, H, seed=1, samples=None):
-    """Run forward + backward and hold every output to the bars of test_attention_fwd_bwd, per head."""
-    scale = D ** -0.5
-    g = torch.Generator(device="cuda").manual_seed(seed)
-    o, o_lo, lse = K.attn_fwd(qkv.view(-1), B, N, H, D, scale)
-    d_o = torch.randn(B * N, H * D, device="cuda", generator=g).to(BF16)
-    dqkv = K.attn_bwd(qkv.view(-1), o, o_lo, lse, d_o, B, N, H, D, scale).view(B, N, 3, H, D)
-    keep = list(range(B)) if samples is None else samples
-    ro, rl, rd = ref_attention(qkv[keep], d_o.view(B, N, H * D)[keep].reshape(-1, H * D), scale)
-    o4, olo4 = o.view(B, N, H, D)[keep], o_lo.view(B, N, H, D)[keep]
-    errs = {"o": worst_head(o4, ro, 2), "o+o_lo": worst_head(o4.double() + olo4.double(), ro, 2),
-            "lse": worst_head(lse[keep], rl, None)}
-    for i, name in enumerate("qkv"):
-        errs["d" + name] = worst_head(dqkv[keep][:, :, i], rd[:, :, i], 2)
-    bars = {"o": 6e-3, "o+o_lo": 3e-3, "lse": 1e-4, "dq": 1.2e-2, "dk": 1.2e-2, "dv": 1.2e-2}
-    for k_, bar in bars.items():
-        assert errs[k_] < bar, (B, N, H, k_, errs)
-    o_inf, no_lo, no_lse = K.attn_fwd(qkv.view(-1), B, N, H, D, scale, train=False)
-    assert no_lo is None and no_lse is None and torch.equal(o_inf, o)
-    return o, lse, dqkv
 
 
 @pytest.mark.parametrize("B,N,H", [(2, 257, 12),     # N % 128 = 1: the last key / query tile holds one row

@@ -384,7 +384,9 @@ def test_attention_fwd_bwd(K, B, N, H, D):
         assert rel(dqkv[:, :, i].float(), dref[:, :, i]) < 1.2e-2, name
 
 
-@pytest.mark.parametrize("B,N,H,R", [(3, 197, 12, 16), (256, 197, 12, 16), (5, 50, 4, 0), (2, 256, 16, 32)])
+@pytest.mark.parametrize("B,N,H,R", [(3, 197, 12, 16), (256, 197, 12, 16), (5, 50, 4, 0), (2, 256, 16, 32),
+                                     (2, 129, 12, 16),      # a second query tile of one row
+                                     (3, 209, 12, 16)])     # N = 209: the backward without the Q/K prefetch
 def test_gemm_delta_epilogue_feeds_attention_backward(K, B, N, H, R):
     """EPI_DELTA: the output projection's dX GEMM (frozen W^T + adapter-transpose segment) also writes
     delta[b,h,n] = sum_d bf16(dO) (O_hi + O_lo) -- bit-for-bit the dO it stores, so it must equal the stand-alone
@@ -456,7 +458,7 @@ def test_merge_adamw_sgemm(K):
     assert rel(K.sgemm(a.t(), a), a.t() @ a) < 1e-5
 
 
-@pytest.mark.parametrize("B,N,H,D", [(2, 197, 3, 64), (1, 257, 2, 80), (2, 33, 2, 64)])
+@pytest.mark.parametrize("B,N,H,D", [(2, 197, 3, 64), (1, 257, 2, 80), (2, 33, 2, 64), (1, 288, 2, 64), (3, 32, 2, 80)])
 def test_fp32_mode_attention_and_gelu(K, B, N, H, D):
     g = torch.Generator(device="cuda").manual_seed(11)
     qkv = torch.randn(B, N, 3, H, D, device="cuda", generator=g)
