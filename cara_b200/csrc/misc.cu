@@ -395,6 +395,7 @@ int merge_launch(const float* W, const float* A, const float* Bf, const float* c
     case 8: merge_kernel<8><<<grid, 128, 0, st>>>(W, A, Bf, cs, out, N, K, w); break;
     case 16: merge_kernel<16><<<grid, 128, 0, st>>>(W, A, Bf, cs, out, N, K, w); break;
     case 32: merge_kernel<32><<<grid, 128, 0, st>>>(W, A, Bf, cs, out, N, K, w); break;
+    case 64: merge_kernel<64><<<grid, 128, 0, st>>>(W, A, Bf, cs, out, N, K, w); break;
     default: return -65;
   }
   return cudaGetLastError() == cudaSuccess ? 0 : -66;

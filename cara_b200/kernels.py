@@ -41,8 +41,14 @@ def _p(t):
     return None if t is None else t.data_ptr()
 
 
+MAX_RANK = 64   # the largest rank the rank-R kernels (skinny, merge) are instantiated for
+
+
 def round_rank(r):
-    return 16 if r <= 16 else 32
+    """The padded rank Rp (16, 32 or 64) the bf16 kernels run a rank-r adapter at."""
+    if r > MAX_RANK:
+        raise ValueError("rank %d > %d is not supported by the bf16 kernels" % (r, MAX_RANK))
+    return 16 if r <= 16 else 32 if r <= 32 else 64
 
 
 _sync_ws = {}
@@ -373,12 +379,12 @@ def assemble_tokens(pe, cls, pos, B, N, Cc):
     return x
 
 
-_MERGE_RANKS = (4, 8, 16, 32)
+_MERGE_RANKS = (4, 8, 16, 32, 64)
 
 
 def merge_weights(W, A, Bf, cs, out=None):
     """W fp32 [N,K], A fp32 [K,R], Bf fp32 [N/S,R], cs fp32 [S,R] -> bf16 [N,K] = W + sum_r (Bf (.) cs) A^T.
-    Any rank up to 32: the factors are zero-padded to the next rank the kernel is instantiated for."""
+    Any rank up to 64: the factors are zero-padded to the next rank the kernel is instantiated for."""
     st = _prep(W)
     N, K = W.shape
     S, R = cs.shape

@@ -12,6 +12,7 @@ from . import _lib as L
 from . import kernels as K
 
 BF16, F32 = torch.bfloat16, torch.float32
+SIDE_RPS = (16, 32)   # padded ranks the projection GEMM's side tiles cover (CARA_SIDE_TILES=1)
 
 
 class FrozenLinear:
@@ -119,12 +120,12 @@ def _cp_linear_fwd(x, fz, bias_eff, ops, epi=L.EPI_NONE, want_pre=True, train=Tr
     """The frozen product + the adapter segment (cara.py:35,57,81,92 without the delta weight).  The rank-R row
     contraction T = x A, Uhat_s = cs_s (.) T that feeds the segment comes from the LayerNorm kernel that produced x
     (``pre``, a filled forward RowsLink), or runs as its own pass (default) or, with CARA_SIDE_TILES=1, as side tiles
-    of the same GEMM launch."""
+    of the same GEMM launch (Rp = 16 / 32; an Rp = 64 projection keeps its own pass)."""
     T = U = None
     if ops is not None and pre is not None and pre.U is not None:
         T, U = pre.T, pre.U
         y = K.gemm_cp(x, fz.w, bias=bias_eff, a1=U, b1=ops.b_ext, ext_slices=ops.slices, epi=epi, want_pre=want_pre)
-    elif ops is not None and not (K.side_tiles and epi == L.EPI_NONE):
+    elif ops is not None and not (K.side_tiles and epi == L.EPI_NONE and ops.rp in SIDE_RPS):
         # default: the row contraction T = x A, Uhat_s = cs_s (.) T as its own HBM-bound pass, then the GEMM
         T, U = K.adapter_rows_fwd(x, ops.a_t2, ops.cs_pad)
         y = K.gemm_cp(x, fz.w, bias=bias_eff, a1=U, b1=ops.b_ext, ext_slices=ops.slices, epi=epi, want_pre=want_pre)
@@ -160,7 +161,7 @@ def _cp_linear_bwd(G, x, fz, ops, T, U, need_dx, need_bias, dgelu_aux=None, sink
         zs = torch.split(z, sizes)
         dcs, dA, dB = zs[0].view(S, Rp), zs[1].view(Kin, Rp), zs[2].view(w, Rp)
         colsum = zs[3] if need_bias else None
-    if dT_pre is not None or not (K.side_tiles and epi == L.EPI_NONE):
+    if dT_pre is not None or not (K.side_tiles and epi == L.EPI_NONE and Rp in SIDE_RPS):
         # the three readers of G run back to back: for the C-wide projections G (77 MB at ViT-B) stays in the 126 MB L2
         # (dT_pre: dThat and dcs already came out of the LayerNorm backward that produced G)
         dT = dT_pre if dT_pre is not None else K.adapter_rows_bwd(G, ops.b_t2, ops.cs_pad, T, dsc=dcs)[0]

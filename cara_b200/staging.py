@@ -131,9 +131,9 @@ def staged(model):
         return cache[1], cache[2]
     dev = P["CP_A1"].device
     R = P["CP_A1"].shape[1]
+    if R > K.MAX_RANK:
+        raise NotImplementedError("rank > %d is not supported by the staged bf16 operands (got %d)" % (K.MAX_RANK, R))
     Rp = K.round_rank(R)
-    if R > 32:
-        raise NotImplementedError("rank > 32 is not supported by the staged bf16 operands (got %d)" % R)
     C = P["CP_A2"].shape[0]
     f = {n: p.float() for n, p in P.items()}
     La, Lm = len(attn), len(mlp)

@@ -121,7 +121,7 @@ CARA_API int cara_ln_bwd_rows(const void* dh, const float* x, const float* mean,
 /* Rank-R side chain.  Precision convention: factor matrices and low-rank activations are bf16 (hi, lo) pairs
  * (x = hi + lo).  A transposed factor operand "Ft2" is bf16 [2*Rp, K] = [hi rows ; lo rows]; a low-rank
  * activation block is bf16 [.., 3*Rp] = [hi | lo | hi], to be multiplied in cara_gemm_cp (K1 = 3*Rp) against
- * an out-side factor laid out [hi | hi | lo].  Rp = rank zero-padded to 16 or 32.
+ * an out-side factor laid out [hi | hi | lo].  Rp = rank zero-padded to 16, 32 or 64.
  *
  * Forward (SURVEY A.1):  T = X A (fp32 [M,Rp]);  Uhat[:, s*3Rp : (s+1)*3Rp] = split(scales[s] (.) T).
  * X bf16 [M,K] (K % 64 == 0); At2 = split(A)^T; scales fp32 [slices,Rp].
