@@ -70,6 +70,8 @@ _SIGS = {
     "cara_adapter_cols": (C.c_int, [_P, C.c_long, C.c_int, C.c_int, _P, C.c_long, C.c_int, C.c_int, _P, _P, _P]),
     "cara_attn_fwd": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, _P]),
     "cara_attn_bwd": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, _P]),
+    "cara_attn_tiled_fwd": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, _P]),
+    "cara_attn_tiled_bwd": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, _P]),
     "cara_debug_read": (C.c_int, [_P, C.c_int]),
     "cara_gelu_f32": (C.c_int, [_P, _P, _P, C.c_long, _P]),
     "cara_attn_f32": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, _P]),

@@ -136,6 +136,25 @@ int cara_attn_bwd(const void* qkv, const void* o, const void* o_lo, const float*
     return fail(-50, "cara_attn_bwd: a precomputed delta (o == NULL) needs D = 64 and delta_ws");
   CARA_RET(cara::attn_bwd_launch(a, CARA_STREAM(stream)), "cara_attn_bwd");
 }
+int cara_attn_tiled_fwd(const void* qkv, void* o, void* o_lo, float* lse, int B, int N, int H, int D, float scale,
+                        void* stream) {
+  if (D != 80 || B <= 0 || N <= 0 || H <= 0 || o == nullptr)
+    return fail(-50, "cara_attn_tiled_fwd: needs D = 80, B, N, H >= 1 and o");
+  cara::AttnArgs a{static_cast<const bf16*>(qkv), static_cast<bf16*>(o), static_cast<bf16*>(o_lo), lse, nullptr,
+                   nullptr, nullptr, B, N, H, D, scale};
+  CARA_RET(cara::attn_fwd_tiled_launch(a, CARA_STREAM(stream)), "cara_attn_tiled_fwd");
+}
+int cara_attn_tiled_bwd(const void* qkv, const void* o, const void* o_lo, const float* lse, const void* d_o, void* dqkv,
+                        float* delta_ws, int B, int N, int H, int D, float scale, void* stream) {
+  if (D != 80 || B <= 0 || N <= 0 || H <= 0)
+    return fail(-50, "cara_attn_tiled_bwd: needs D = 80 and B, N, H >= 1");
+  if (o == nullptr || o_lo == nullptr || delta_ws == nullptr)
+    return fail(-50, "cara_attn_tiled_bwd: needs o, o_lo and delta_ws (delta is computed here, not taken precomputed)");
+  cara::AttnArgs a{static_cast<const bf16*>(qkv), static_cast<bf16*>(const_cast<void*>(o)),
+                   static_cast<bf16*>(const_cast<void*>(o_lo)), const_cast<float*>(lse),
+                   static_cast<const bf16*>(d_o), static_cast<bf16*>(dqkv), delta_ws, B, N, H, D, scale};
+  CARA_RET(cara::attn_bwd_tiled_launch(a, CARA_STREAM(stream)), "cara_attn_tiled_bwd");
+}
 int cara_gelu_f32(const float* dy, const float* x, float* out, long n, void* stream) {
   CARA_RET(cara::gelu_f32_launch(dy, x, out, n, CARA_STREAM(stream)), "cara_gelu_f32");
 }

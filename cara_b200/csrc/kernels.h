@@ -102,6 +102,9 @@ int attn_delta_launch(const AttnArgs& a, cudaStream_t st);
 // key-tiled tcgen05 variants (attention_long.cu): 0 = launched, 1 = shape not covered (D != 64 or N <= 256), < 0 = error
 int attn_fwd_long_launch(const AttnArgs& a, cudaStream_t st);
 int attn_bwd_long_launch(const AttnArgs& a, cudaStream_t st);
+// key-tiled mma.sync kernels for D = 80 at any N (attention_tiled.cu): 0 = launched, < 0 = error (D != 80 included)
+int attn_fwd_tiled_launch(const AttnArgs& a, cudaStream_t st);
+int attn_bwd_tiled_launch(const AttnArgs& a, cudaStream_t st);
 
 // fp32.cu: fp32 parity mode (exact-erf GELU forward / backward, attention core forward / backward in SIMT fp32)
 int gelu_f32_launch(const float* dy, const float* x, float* out, long n, cudaStream_t st);

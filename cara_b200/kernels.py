@@ -334,6 +334,34 @@ def attn_bwd(qkv, o, o_lo, lse, d_o, B, N, H, D, scale, delta=None):
     return dqkv
 
 
+# The largest N the whole-head D = 80 kernels (cara_attn_fwd / cara_attn_bwd) take: the head's tiles must fit in shared
+# memory.  Above them ops.AttnCoreFunction runs the key-tiled kernels (cara_attn_tiled_fwd / _bwd), which take any N.
+D80_WHOLE_HEAD_MAX_N = {"fwd": 432, "bwd": 320}
+
+
+def attn_tiled_fwd(qkv, B, N, H, D, scale, train=True):
+    """``attn_fwd`` on the key-tiled D = 80 kernels (any N): -> (o, o_lo, lse); o_lo / lse are None when train is False."""
+    st = _prep(qkv)
+    assert qkv.dtype == BF16 and qkv.is_contiguous() and qkv.numel() == B * N * 3 * H * D
+    o = torch.empty((B * N, H * D), device=qkv.device, dtype=BF16)
+    o_lo = torch.empty_like(o) if train else None
+    lse = torch.empty((B, H, N), device=qkv.device, dtype=F32) if train else None
+    L.check(L.lib().cara_attn_tiled_fwd(qkv.data_ptr(), o.data_ptr(), _p(o_lo), _p(lse), B, N, H, D, scale, st),
+            "cara_attn_tiled_fwd")
+    return o, o_lo, lse
+
+
+def attn_tiled_bwd(qkv, o, o_lo, lse, d_o, B, N, H, D, scale):
+    """``attn_bwd`` on the key-tiled D = 80 kernels (any N); always runs its own delta pre-pass (o and o_lo needed)."""
+    st = _prep(qkv)
+    assert d_o.is_contiguous() and d_o.dtype == BF16
+    dqkv = torch.empty_like(qkv)
+    delta = torch.empty((B, H, N), device=qkv.device, dtype=F32)
+    L.check(L.lib().cara_attn_tiled_bwd(qkv.data_ptr(), _p(o), _p(o_lo), lse.data_ptr(), d_o.data_ptr(), dqkv.data_ptr(),
+                                        delta.data_ptr(), B, N, H, D, scale, st), "cara_attn_tiled_bwd")
+    return dqkv
+
+
 def gelu_f32(x, dy=None):
     """fp32 mode: GELU(x) (dy None) or dy * GELU'(x), exact erf."""
     st = _prep(x)

@@ -282,12 +282,20 @@ class AttnLink:
         self.o_lo = self.shape = self.delta = None
 
 
+def _d80_tiled(D, N, direction):
+    """D = 80 above the whole-head kernels' shared-memory limit runs on the key-tiled kernels (any N).  Below it the
+    whole-head kernels keep running, so ViT-H/14 at 224 px launches what it always did; between the two limits
+    (320 < N <= 432) a whole-head forward feeds a tiled backward."""
+    return D == 80 and N > K.D80_WHOLE_HEAD_MAX_N[direction]
+
+
 class AttnCoreFunction(torch.autograd.Function):
     """softmax(q k^T D^-1/2) v on the fused projection's [B,N,3,H,D] output (cara.py:44-48)."""
 
     @staticmethod
     def forward(ctx, qkv, B, N, H, D, scale, link=None):
-        o, o_lo, lse = K.attn_fwd(qkv, B, N, H, D, scale, train=ctx.needs_input_grad[0])
+        fwd = K.attn_tiled_fwd if _d80_tiled(D, N, "fwd") else K.attn_fwd
+        o, o_lo, lse = fwd(qkv, B, N, H, D, scale, train=ctx.needs_input_grad[0])
         ctx.dims = (B, N, H, D, scale)
         ctx.link = link
         if link is not None and o_lo is not None:
@@ -302,6 +310,9 @@ class AttnCoreFunction(torch.autograd.Function):
         delta = None
         if ctx.link is not None:
             delta, ctx.link.delta = ctx.link.delta, None
+        if _d80_tiled(D, N, "bwd"):                        # no EPI_DELTA at D = 80: delta is None here
+            return (K.attn_tiled_bwd(qkv, o, o_lo, lse, d_o.contiguous(), B, N, H, D, scale),
+                    None, None, None, None, None, None)
         return (K.attn_bwd(qkv, o, o_lo, lse, d_o.contiguous(), B, N, H, D, scale, delta=delta),
                 None, None, None, None, None, None)
 

@@ -145,16 +145,29 @@ CARA_API int cara_adapter_cols(const void* X, long ldx, int M, int Kc, const voi
  * For training also pass lse [B,H,N] fp32 (base-2 log-sum-exp of the scaled scores) and o_lo [B,N,H,D] bf16
  * (the rounding residual of o: o_fp32 = o + o_lo), both consumed by cara_attn_bwd; NULL for inference.
  * D in {64,80}.  D = 64 runs on tcgen05 at every N (N <= 256: one head per CTA pass; N > 256: 128-key tiles);
- * D = 80 runs on mma.sync with the whole head in shared memory: N <= 432, larger N returns an error. */
+ * D = 80 runs on mma.sync with the whole head in shared memory: N <= 432, larger N returns an error (cara_attn_tiled_fwd
+ * below runs D = 80 at any N). */
 CARA_API int cara_attn_fwd(const void* qkv, void* o, void* o_lo, float* lse, int B, int N, int H, int D,
                            float scale, void* stream);
 /* delta_ws: caller-provided fp32 workspace [B,H,N] (rowsum(dO (.) O), written by a streaming pre-pass).
  * o == NULL (D = 64 only, any N): delta_ws already holds it -- written by the output projection's dX GEMM
  * (cara_gemm_cp, epi = CARA_EPI_DELTA) -- and the pre-pass is skipped.
  * D = 64 runs on tcgen05 at every N; D = 80 runs on mma.sync with the whole head in shared memory: N <= 320, larger N
- * returns an error.  Neither uses atomics: dqkv is bit-identical from run to run. */
+ * returns an error (cara_attn_tiled_bwd below runs D = 80 at any N).  Neither uses atomics: dqkv is bit-identical from
+ * run to run. */
 CARA_API int cara_attn_bwd(const void* qkv, const void* o, const void* o_lo, const float* lse, const void* d_o,
                            void* dqkv, float* delta_ws, int B, int N, int H, int D, float scale, void* stream);
+/* The same two calls for D = 80 at any N >= 1 (ViT-H/14 above 224 px), on key-tiled mma.sync kernels: a CTA holds a
+ * 128-query (forward), 64-query (dQ) or 64-key (dK/dV) tile and streams the other operand through a two-stage ring of
+ * 64-row windows, so shared memory does not grow with N.  Arguments, layouts and outputs are those of cara_attn_fwd /
+ * cara_attn_bwd; the backward always runs its own delta pre-pass into delta_ws (o, o_lo and delta_ws are required).
+ * Where the whole-head D = 80 calls above also run (forward N <= 432, backward N <= 320), the results are bit-identical
+ * to theirs, and a whole-head forward may feed a tiled backward.  No atomics: dqkv is bit-identical from run to run.
+ * D != 80, B, N or H <= 0, and a NULL o (or, backward, o_lo / delta_ws) return an error before any launch. */
+CARA_API int cara_attn_tiled_fwd(const void* qkv, void* o, void* o_lo, float* lse, int B, int N, int H, int D,
+                                 float scale, void* stream);
+CARA_API int cara_attn_tiled_bwd(const void* qkv, const void* o, const void* o_lo, const float* lse, const void* d_o,
+                                 void* dqkv, float* delta_ws, int B, int N, int H, int D, float scale, void* stream);
 /* Profiling aid: copies up to n device-side cycle stamps recorded by the attention kernels (debug builds of the
  * kernels only write them for CTA 0); returns the number of values copied. */
 CARA_API int cara_debug_read(long long* out, int n);
